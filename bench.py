@@ -5,7 +5,7 @@ One "step" = one pass of the hot path (the batched rx loop: per-stream frame
 search + tone correlation + rx state machine, src/minimodem.c:1137-1463 over
 src/fsk.c:449-538) over one batch of synthetic streams.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 N>1 is launched by torchrun (one rank per GPU); streams shard across ranks with
 no data-path collective (weak scaling: every rank demodulates its own batch);
@@ -40,6 +40,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True          # no __pycache__ in the tree: it may be read-only
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -73,6 +74,8 @@ def parse():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-configs", action="store_true")
     ap.add_argument("--only-config", default="", help="run only the `configs` entries whose key contains this")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the frame records and stream states of the headline's last timed step to DIR/*.npy")
     return ap.parse_args()
 
 
@@ -417,6 +420,27 @@ def time_rx(torch, dist, world, dev, eng, x, n, max_frames, frames, states, step
     return ms_step, ms_kernel, clocks
 
 
+def dump_outputs(mm, torch, out_dir, frames, states, budget=60_000_000):
+    """What rx_batch handed its caller in the last timed step, as float64 arrays (exact for every field):
+    DIR/frames_<field>.npy [k, max_frames] per frame-record field, zero past each stream's nframes (those
+    slots hold no record), DIR/states_<field>.npy [k] per stream-state field, and DIR/streams.npy, the
+    rows they belong to -- all streams, or a fixed seeded sample of them that keeps the files under `budget`."""
+    S, max_frames = frames.shape[0], frames.shape[1]
+    per_stream = 8 * (1 + max_frames * len(mm.FRAME_DTYPE.names) + len(mm.STATE_DTYPE.names))
+    k = min(S, max(1, budget // per_stream))
+    rows = np.arange(S) if k == S else np.sort(np.random.default_rng(20260922).choice(S, k, replace=False))
+    sel = torch.from_numpy(rows).to(frames.device)
+    fr = mm.frames_to_numpy(frames.index_select(0, sel))
+    st = mm.states_to_numpy(states.index_select(0, sel))
+    valid = np.arange(max_frames)[None, :] < st["nframes"].astype(np.int64)[:, None]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "streams.npy"), rows.astype(np.float64))
+    for f in mm.FRAME_DTYPE.names:
+        np.save(os.path.join(out_dir, "frames_%s.npy" % f), np.where(valid, fr[f], 0).astype(np.float64))
+    for f in mm.STATE_DTYPE.names:
+        np.save(os.path.join(out_dir, "states_%s.npy" % f), st[f].astype(np.float64))
+
+
 def summarize(mm, torch, dist, world, dev, wl, frames, states, ms_step, ms_kernel, clean, peak):
     """Per-workload result block: throughput, roofline fraction, device-side statistics, decode check."""
     S, n = wl.S, wl.n
@@ -499,6 +523,8 @@ def run_ours(a):
     ms_step, ms_kernel, clocks = time_rx(torch, dist, world, dev, eng, x, n, max_frames, frames, states,
                                          a.steps, a.warmup, sampler)
     launches = mm.launch_count() - launches0 - a.warmup
+    if a.dump_outputs and rank == 0:
+        dump_outputs(mm, torch, a.dump_outputs, frames, states)
     head = summarize(mm, torch, dist, world, dev, wl, frames, states, ms_step, ms_kernel,
                      clean=not (a.awgn or a.offset), peak=peak)
     st = mm.states_to_numpy(states)

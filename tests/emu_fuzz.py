@@ -164,29 +164,22 @@ def test_second_batch_of_option_vectors(case):
 
 
 @pytest.mark.parametrize("seed", range(40))
-def test_batched_kernels_print_what_the_reference_cli_prints(seed, tmp_path):
+def test_batched_kernels_print_what_the_reference_cli_prints(seed):
     """Closing the loop without the oracle in between: a random invocation goes through the
-    unmodified reference CLI (transmit, then receive), and the same audio through rx_batch +
-    decode_batch on the emulated kernels; the text must be the CLI's stdout.  (Where the reference's
-    sample ring makes it read stale samples -- slow modes, DESIGN.md 5 item 2 -- the oracle's two
-    modes already differ and the case is skipped.)"""
-    import os
-    import subprocess
-    import sys
-    sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
-    from make_golden import read_wav
+    unmodified reference CLI (transmit, then receive; its recorded answers where oracle/_ref is not
+    built), and the same audio through rx_batch + decode_batch on the emulated kernels; the text must
+    be the CLI's stdout.  (Where the reference's sample ring makes it read stale samples -- slow
+    modes, DESIGN.md 5 item 2 -- the oracle's two modes already differ and the case is skipped.)"""
+    import hashlib
     from test_oracle_fuzz_vs_cli import random_invocation
-    if not orc.have_ref() or not os.path.exists(orc.REF_CLI):
-        pytest.skip("needs the reference CLI (oracle/_ref)")
     rng = np.random.default_rng(12000 + seed)
     mode, kw, tx_args, rx_args, flt, vol = random_invocation(rng)
     text = bytes(rng.integers(32, 127, int(rng.integers(4, 30)), dtype=np.uint8)) + b"\n"
-    wav = str(tmp_path / "x.wav")
-    subprocess.run([orc.REF_CLI, "--tx", "--file", wav] + tx_args, input=text, check=True)
-    ref = subprocess.run([orc.REF_CLI, "--rx", "--file", wav] + rx_args, stdout=subprocess.PIPE,
-                         stderr=subprocess.PIPE, check=True)
-    audio, rate, _ = read_wav(wav)
+    ref = orc.ref_cli(tx_args, rx_args, text)
     m = orc.Mode(mode, **kw)
+    # the audio the reference's transmitter wrote, from the oracle's bit-exact restatement of it
+    audio = orc.tx_words(m, orc.ref_encode("ascii8", text) & ((1 << m.n_data_bits) - 1), vol, 4096, flt)
+    assert hashlib.sha256(audio.tobytes()).hexdigest() == ref["audio_sha256"], tx_args
     lit = orc.rx_run(m, audio, literal=True)["frames"]
     flat = orc.rx_run(m, audio, literal=False)["frames"]
     if [f[:1] + f[3:5] for f in lit] != [f[:1] + f[3:5] for f in flat]:
@@ -199,4 +192,4 @@ def test_batched_kernels_print_what_the_reference_cli_prints(seed, tmp_path):
     out, cnt = eng.decode_batch(mm.decoder_for_mode(mode, m.n_data_bits), frames, states)
     o, c = out.cpu().numpy(), cnt.cpu().numpy()
     for s in range(2):
-        assert bytes(o[s, :c[s]]) == ref.stdout, (rx_args, bytes(o[s, :c[s]])[:40], ref.stdout[:40])
+        assert bytes(o[s, :c[s]]) == ref["stdout"], (rx_args, bytes(o[s, :c[s]])[:40], ref["stdout"][:40])

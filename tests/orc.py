@@ -3,12 +3,21 @@ CPU restatement) and for oracle/_ref/libfsk_ref.so (the unmodified reference
 src/fsk.c + databits decoders compiled in place).  Only tests/, bench.py's
 cpu_baseline / --impl reference legs and __graft_entry__.smoke() import this.
 
+Where oracle/_ref is not built, the reference's answers to the tests' inputs come
+from tests/golden/reference_results.json (see `recorded`).
+
 Also holds an independent Python restatement of the reference's mode presets
 (src/minimodem.c:819-965) used to cross-check the product's host-side presets.
 """
+import atexit
+import base64
 import ctypes as C
+import hashlib
+import json
 import os
 import subprocess
+import sys
+import tempfile
 
 import numpy as np
 
@@ -21,6 +30,8 @@ LIBREF_DFTI = os.path.join(ORACLE_DIR, "_ref", "libfsk_ref_dfti.so")
 REF_CLI = os.path.join(ORACLE_DIR, "_ref", "minimodem_ref")
 REF_CLI_TRACE = os.path.join(ORACLE_DIR, "_ref", "minimodem_ref_trace")
 REFERENCE_SRC = "/root/reference"
+GOLDEN_DIR = os.path.join(ROOT, "tests", "golden")
+RECORDED = os.path.join(GOLDEN_DIR, "reference_results.json")
 
 f32 = np.float32
 
@@ -43,6 +54,101 @@ def build_ref():
 
 def have_ref():
     return os.path.exists(LIBREF)
+
+
+# --------------------------------------------------------------------------
+# recorded answers of the unmodified reference
+# --------------------------------------------------------------------------
+_store = None
+_new = {}
+
+
+def _read_store():
+    if not os.path.exists(RECORDED):
+        return {}
+    with open(RECORDED) as f:
+        return json.load(f)
+
+
+def _load_store():
+    global _store
+    if _store is None:
+        _store = _read_store()
+        if os.environ.get("FSK_RECORD_REFERENCE") == "1":
+            atexit.register(_save_store)
+    return _store
+
+
+def _save_store():
+    """Adds this process's answers to the file (other processes may have added theirs meanwhile)."""
+    if _new:
+        store = _read_store()
+        store.update(_new)
+        with open(RECORDED, "w") as f:
+            f.write("{\n" + ",\n".join("%s:%s" % (json.dumps(k), json.dumps(store[k], separators=(",", ":")))
+                                       for k in sorted(store)) + "\n}\n")
+
+
+def record_key(*parts):
+    """A stable name for one question put to the reference: its function and every input, byte for byte."""
+    h = hashlib.sha256()
+    for p in parts:
+        if isinstance(p, np.ndarray):
+            b = p.dtype.str.encode() + repr(p.shape).encode() + np.ascontiguousarray(p).tobytes()
+        elif isinstance(p, (bytes, bytearray)):
+            b = bytes(p)
+        elif isinstance(p, (float, np.floating)):
+            b = np.float64(p).tobytes()
+        else:
+            b = repr(p).encode()
+        h.update(len(b).to_bytes(8, "little") + b)
+    return h.hexdigest()[:32]
+
+
+def recorded(key, live):
+    """The reference's answer to the question `key`.  Where oracle/_ref is built, `live()` asks the
+    compiled reference (and FSK_RECORD_REFERENCE=1 writes the answer to tests/golden/reference_results.json);
+    elsewhere the answer comes from that file.  A question it has no answer for is an error: the input
+    the test put to the reference is not the one it was recorded with."""
+    store = _load_store()
+    if have_ref():
+        value = live()
+        if os.environ.get("FSK_RECORD_REFERENCE") == "1":
+            _new[key] = value
+        return value
+    assert key in store, "no recorded reference answer for this input (%s); oracle/_ref is not built" % key
+    return store[key]
+
+
+class RecordedBytes:
+    """A long output of the reference, recorded as its length and sha256: equal to exactly those bytes."""
+
+    def __init__(self, n, sha256):
+        self.n, self.sha256 = n, sha256
+
+    def __eq__(self, other):
+        if isinstance(other, RecordedBytes):
+            return (self.n, self.sha256) == (other.n, other.sha256)
+        return (isinstance(other, (bytes, bytearray)) and len(other) == self.n
+                and hashlib.sha256(other).hexdigest() == self.sha256)
+
+    __hash__ = None
+
+    def __len__(self):
+        return self.n
+
+    def __repr__(self):
+        return "<%d bytes of reference output, sha256 %s>" % (self.n, self.sha256)
+
+
+def _enc_bytes(b, verbatim=256):
+    if len(b) <= verbatim:
+        return base64.b64encode(bytes(b)).decode()
+    return {"len": len(b), "sha256": hashlib.sha256(b).hexdigest()}
+
+
+def _dec_bytes(v):
+    return base64.b64decode(v) if isinstance(v, str) else RecordedBytes(v["len"], v["sha256"])
 
 
 # --------------------------------------------------------------------------
@@ -541,60 +647,135 @@ def ref_dfti():
 
 
 class RefPlan:
-    """fsk_plan of the unmodified reference (src/fsk.c:33)."""
+    """fsk_plan of the unmodified reference (src/fsk.c:33); recorded answers where oracle/_ref is not built."""
 
     def __init__(self, sample_rate, f_mark, f_space, bw):
-        self.h = ref().fsk_plan_new(sample_rate, f_mark, f_space, bw)
-        if not self.h:
-            raise ValueError("fsk_plan_new failed")
+        self.args = tuple(float(f32(x)) for x in (sample_rate, f_mark, f_space, bw))
+        self.h = None
+        if have_ref():
+            self.h = ref().fsk_plan_new(sample_rate, f_mark, f_space, bw)
+            if not self.h:
+                raise ValueError("fsk_plan_new failed")
 
     def __del__(self):
         try:
-            ref().fsk_plan_destroy(self.h)
+            if self.h:
+                ref().fsk_plan_destroy(self.h)
         except Exception:
             pass
 
     def find_frame(self, samples, frame_nsamples, try_first, try_max, try_step, limit, expect):
-        bits, ampl, start = C.c_ulonglong(0), C.c_float(0), C.c_uint(0)
         if isinstance(expect, str):
             expect = expect.encode()
-        c = ref().fsk_find_frame(self.h, fptr(samples), frame_nsamples, try_first, try_max, try_step,
-                                 limit, expect, C.byref(bits), C.byref(ampl), C.byref(start))
-        return f32(c), bits.value, f32(ampl.value), start.value
+        args = (int(frame_nsamples), int(try_first), int(try_max), int(try_step), float(f32(limit)), bytes(expect))
+
+        def live():
+            bits, ampl, start = C.c_ulonglong(0), C.c_float(0), C.c_uint(0)
+            c = ref().fsk_find_frame(self.h, fptr(samples), frame_nsamples, try_first, try_max, try_step,
+                                     limit, expect, C.byref(bits), C.byref(ampl), C.byref(start))
+            return [float(f32(c)), int(bits.value), float(f32(ampl.value)), int(start.value)]
+        c, bits, ampl, start = recorded(record_key("fsk_find_frame", self.args, samples, args), live)
+        return f32(c), bits, f32(ampl), start
+
+    def detect_carrier(self, samples, nsamples, threshold):
+        def live():
+            fn = ref().fsk_detect_carrier
+            fn.argtypes = [C.c_void_p, C.POINTER(C.c_float), C.c_uint, C.c_float]
+            fn.restype = C.c_int
+            return int(fn(self.h, fptr(samples), nsamples, threshold))
+        return recorded(record_key("fsk_detect_carrier", self.args, samples, int(nsamples), float(f32(threshold))),
+                        live)
 
 
 def ref_encode(decoder, data):
     """bytes -> frame data words through the reference's databits encoder."""
-    L = ref()
-    enc = L.baudot_encode if decoder == "baudot" else L.databits_encode_ascii8
-    words = []
-    buf = (C.c_uint * 2)()
-    for ch in data:
-        n = enc(buf, C.c_char(bytes([ch])))
-        words.extend(buf[i] for i in range(n))
-    return np.array(words, np.uint32)
+    def live():
+        L = ref()
+        enc = L.baudot_encode if decoder == "baudot" else L.databits_encode_ascii8
+        words = []
+        buf = (C.c_uint * 2)()
+        for ch in data:
+            n = enc(buf, C.c_char(bytes([ch])))
+            words.extend(int(buf[i]) for i in range(n))
+        return words
+    return np.array(recorded(record_key("databits_encode", decoder, bytes(data)), live), np.uint32)
+
+
+REF_DECODERS = {"ascii8": "databits_decode_ascii8", "baudot": "databits_decode_baudot",
+                "callerid": "databits_decode_callerid", "binary": "databits_decode_binary",
+                "uic-ground": "databits_decode_uic_ground", "uic-train": "databits_decode_uic_train"}
+
+
+def ref_decode_words(kind, n_data_bits, words, resets, L=None):
+    """data words -> output bytes through the reference's databits decoder `kind`, with a decoder reset
+    before word i where resets[i].  L: the reference library to call (default: oracle/_ref/libfsk_ref.so)."""
+    words = np.ascontiguousarray(words, np.uint64)
+    resets = np.ascontiguousarray(resets, np.bool_)
+
+    def live():
+        fn = getattr(L or ref(), REF_DECODERS[kind])
+        fn.argtypes = [C.c_char_p, C.c_uint, C.c_ulonglong, C.c_uint]
+        fn.restype = C.c_uint
+        buf = C.create_string_buffer(8192)
+        out = bytearray()
+        for w, r in zip(words, resets):
+            if r:
+                fn(None, 0, 0, 0)
+            n = fn(buf, 8192, int(w), n_data_bits)
+            out += buf.raw[:n]
+        return _enc_bytes(out)
+    return _dec_bytes(recorded(record_key("databits_decode", kind, int(n_data_bits), words, resets), live))
 
 
 def ref_decode(mode, frames, decoder=None):
     """frame records -> output bytes through the reference's databits decoder,
     following src/minimodem.c:1351 (reset on acquire) and :1415-1446."""
-    L = ref()
-    name = decoder or mode.decoder
-    fn = {"ascii8": L.databits_decode_ascii8, "baudot": L.databits_decode_baudot,
-          "callerid": L.databits_decode_callerid, "binary": L.databits_decode_binary,
-          "uic-ground": L.databits_decode_uic_ground, "uic-train": L.databits_decode_uic_train}[name]
-    out = bytearray()
-    buf = C.create_string_buffer(4096)
+    words, resets = [], []
+    reset = False
     for fr in frames:
         bits, acquired = fr[0], fr[4]
-        if acquired:
-            fn(None, 0, 0, 0)
+        reset = reset or bool(acquired)
         data = databits(mode, bits)
-        if mode.do_rx_sync and data == mode.sync_byte:      # :1436-1439
+        if mode.do_rx_sync and data == mode.sync_byte:      # :1436-1439 (a reset there acts on the next word)
             continue
-        n = fn(buf, 4096, data, mode.n_data_bits)
-        out += buf.raw[:n]
-    return bytes(out)
+        words.append(data)
+        resets.append(reset)
+        reset = False
+    return ref_decode_words(decoder or mode.decoder, mode.n_data_bits, words, resets)
+
+
+def ref_cli(tx_args, rx_args, text):
+    """The unmodified reference CLI: `--tx tx_args` writes `text` to a WAV file, `--rx rx_args` reads it back.
+    Returns what the tests compare with: the length and sha256 of the float32 samples the receiver saw, its
+    stdout and its NOCARRIER stat lines."""
+    def live():
+        if GOLDEN_DIR not in sys.path:
+            sys.path.insert(0, GOLDEN_DIR)
+        from make_golden import read_wav
+        with tempfile.TemporaryDirectory() as d:
+            wav = os.path.join(d, "x.wav")
+            subprocess.run([REF_CLI, "--tx", "--file", wav] + list(tx_args), input=text, check=True)
+            r = subprocess.run([REF_CLI, "--rx", "--file", wav] + list(rx_args), stdout=subprocess.PIPE,
+                               stderr=subprocess.PIPE, check=True)
+            audio, _, _ = read_wav(wav)
+        return {"audio_len": int(audio.size),
+                "audio_sha256": hashlib.sha256(np.ascontiguousarray(audio, np.float32).tobytes()).hexdigest(),
+                "stdout": _enc_bytes(r.stdout),
+                "nocarrier": [ln.strip() for ln in r.stderr.decode().splitlines() if ln.startswith("### NOCARRIER")]}
+    v = recorded(record_key("minimodem", list(tx_args), list(rx_args), bytes(text)), live)
+    return dict(v, stdout=_dec_bytes(v["stdout"]))
+
+
+def ref_cli_tx_image(tx_args, text, keep=256):
+    """The first `keep` bytes and the length of the WAV file the reference CLI's `--tx tx_args` writes for `text`."""
+    def live():
+        with tempfile.TemporaryDirectory() as d:
+            wav = os.path.join(d, "t.wav")
+            subprocess.run([REF_CLI, "--tx", "--file", wav] + list(tx_args), input=text, check=True)
+            image = open(wav, "rb").read()
+        return {"head": _enc_bytes(image[:keep]), "len": len(image)}
+    v = recorded(record_key("minimodem_tx_image", list(tx_args), bytes(text), keep), live)
+    return _dec_bytes(v["head"]), v["len"]
 
 
 def rx_many(mode, samples, nsamples=None, nthreads=1, kind="port"):

@@ -28,39 +28,19 @@ _priv = None
 
 
 def private_ref(tmp_path_factory):
+    """lib: the private copy, or None where oracle/_ref is not built (the decoders' recorded answers stand in)."""
     global _priv
     if _priv is None:
-        d = tmp_path_factory.mktemp("refcopy")
-        path = os.path.join(str(d), "libfsk_ref_private.so")
-        shutil.copy(orc.LIBREF, path)
-        L = C.CDLL(path)
-        for name in ("databits_decode_ascii8", "databits_decode_baudot", "databits_decode_callerid",
-                     "databits_decode_binary", "databits_decode_uic_ground", "databits_decode_uic_train"):
-            fn = getattr(L, name)
-            fn.argtypes = [C.c_char_p, C.c_uint, C.c_ulonglong, C.c_uint]
-            fn.restype = C.c_uint
+        L = None
+        if orc.have_ref():
+            d = tmp_path_factory.mktemp("refcopy")
+            path = os.path.join(str(d), "libfsk_ref_private.so")
+            shutil.copy(orc.LIBREF, path)
+            L = C.CDLL(path)
         _priv = dict(lib=L, state=orc.DecoderState())      # our state with the same history
     return _priv
 
 
-REF_FN = {"ascii8": "databits_decode_ascii8", "binary": "databits_decode_binary",
-          "baudot": "databits_decode_baudot", "callerid": "databits_decode_callerid",
-          "uic-ground": "databits_decode_uic_ground", "uic-train": "databits_decode_uic_train"}
-
-
-def ref_words(L, kind, n_data_bits, words, resets):
-    fn = getattr(L, REF_FN[kind])
-    buf = C.create_string_buffer(8192)
-    out = bytearray()
-    for w, r in zip(words, resets):
-        if r:
-            fn(None, 0, 0, 0)
-        n = fn(buf, 8192, int(w), n_data_bits)
-        out += buf.raw[:n]
-    return bytes(out)
-
-
-@pytest.mark.ref
 @pytest.mark.parametrize("kind,nbits", [("ascii8", 8), ("ascii8", 7), ("binary", 8), ("binary", 5), ("binary", 39),
                                         ("baudot", 5), ("uic-ground", 39), ("uic-train", 39)])
 def test_words_against_reference_decoders(kind, nbits, tmp_path_factory):
@@ -83,7 +63,7 @@ def test_words_against_reference_decoders(kind, nbits, tmp_path_factory):
     resets[0] = True
     st = P["state"]
     got = orc.decode_words(kind, nbits, words, resets, state=st)
-    want = ref_words(P["lib"], kind, nbits, words, resets)
+    want = orc.ref_decode_words(kind, nbits, words, resets, L=P["lib"])
     assert got == want
 
 
@@ -116,7 +96,6 @@ CRAFTED = [
 ]
 
 
-@pytest.mark.ref
 def test_callerid_against_reference_decoder(tmp_path_factory):
     P = private_ref(tmp_path_factory)
     rng = np.random.default_rng(7)
@@ -144,7 +123,7 @@ def test_callerid_against_reference_decoder(tmp_path_factory):
     resets = rng.random(words.size) < 0.003
     resets[0] = True
     got = orc.decode_words("callerid", 8, words, resets, state=P["state"])
-    want = ref_words(P["lib"], "callerid", 8, words, resets)
+    want = orc.ref_decode_words("callerid", 8, words, resets, L=P["lib"])
     assert got == want
     assert got.count(b"CALLER-ID\n") > 300
     import minimodem_b200 as mm

@@ -135,14 +135,13 @@ def test_rx_batch_on_reference_vectors(case):
     (recs,), st = rx_on_gpu(eng, [a])
     got = as_oracle_frames(recs)
     compare_frames(got, want["frames"], case["name"])
-    if orc.have_ref():
-        # byte-identical decode, the reference's own pass criterion (tests/self-test: cmp)
-        frames = got
-        if case["rx_one"]:          # --rx-one: stop at the first carrier drop (:1310)
-            nacq = [i for i, f in enumerate(frames) if f[4]]
-            if len(nacq) > 1:
-                frames = frames[:nacq[1]]
-        assert orc.ref_decode(rx, frames, decoder=refcases.decoder_of(case, rx)) == bytes(g["stdout"])
+    # byte-identical decode, the reference's own pass criterion (tests/self-test: cmp)
+    frames = got
+    if case["rx_one"]:          # --rx-one: stop at the first carrier drop (:1310)
+        nacq = [i for i, f in enumerate(frames) if f[4]]
+        if len(nacq) > 1:
+            frames = frames[:nacq[1]]
+    assert orc.ref_decode(rx, frames, decoder=refcases.decoder_of(case, rx)) == bytes(g["stdout"])
     # stat line (the -P tests grep it for "confidence=inf ... (rate perfect)")
     reps = reports_of(recs, st[0])
     compare_reports(reps, want["reports"], case["name"])
@@ -259,8 +258,7 @@ def test_dropin_find_frame_behind_the_rx_loop(name):
     for i, c in enumerate(got["calls"]):
         assert c[7] == int(cb_[i]) and c[9] == int(cu[i, 4]), (i, c)
         assert gu.close(c[6], cf[i, 1], cond=gu.CONF_COND) and gu.close(c[8], cf[i, 2]), (i, c, cf[i])
-    if orc.have_ref():
-        assert orc.ref_decode(rx, got["frames"]) == bytes(g["stdout"])
+    assert orc.ref_decode(rx, got["frames"]) == bytes(g["stdout"])
     plan.destroy()
 
 
@@ -271,15 +269,11 @@ def test_dropin_detect_carrier_and_bandshift():
     x = (0.8 * np.sin(2 * np.pi * 2200 * t / 48000)).astype(np.float32)
     assert plan.detect_carrier(x, 0.001) == 11          # 2200 Hz / 200 Hz bands
     assert plan.detect_carrier(np.zeros(n, np.float32), 0.001) == -1
-    if orc.have_ref():
-        rp = orc.RefPlan(48000, 1200, 2200, 200)
-        rng = np.random.default_rng(5)
-        for _ in range(8):
-            y = (x * rng.uniform(0.1, 1) + 0.05 * rng.standard_normal(n)).astype(np.float32)
-            want = orc.ref().fsk_detect_carrier
-            want.argtypes = [C.c_void_p, C.POINTER(C.c_float), C.c_uint, C.c_float]
-            want.restype = C.c_int
-            assert plan.detect_carrier(y, 0.001) == want(rp.h, orc.fptr(y), n, 0.001)
+    rp = orc.RefPlan(48000, 1200, 2200, 200)
+    rng = np.random.default_rng(5)
+    for _ in range(8):
+        y = (x * rng.uniform(0.1, 1) + 0.05 * rng.standard_normal(n)).astype(np.float32)
+        assert plan.detect_carrier(y, 0.001) == rp.detect_carrier(y, n, 0.001)
     plan.set_tones_by_bandshift(11, -5)                 # src/fsk.c:584-598
     assert (plan.b_mark, plan.b_space) == (11, 6)
     assert (plan.f_mark, plan.f_space) == (2200.0, 1200.0)
@@ -309,12 +303,7 @@ def test_detect_carrier_batch(rate, bw, n):
     got = mm.detect_carrier_batch(fftsize, d, n, 0.05, offset=torch.from_numpy(off).to(dev()))
     torch.cuda.synchronize()
     got = got.cpu().numpy()
-    want_fn = None
-    if orc.have_ref():
-        rp = orc.RefPlan(rate, plan.f_mark, plan.f_space, bw)
-        want_fn = orc.ref().fsk_detect_carrier
-        want_fn.argtypes = [C.c_void_p, C.POINTER(C.c_float), C.c_uint, C.c_float]
-        want_fn.restype = C.c_int
+    rp = orc.RefPlan(rate, plan.f_mark, plan.f_space, bw)
     for s in range(nstreams):
         w = np.ascontiguousarray(x[s, off[s]:off[s] + n])
         assert got[s] == plan.detect_carrier(w, 0.05), s
@@ -323,13 +312,12 @@ def test_detect_carrier_batch(rate, bw, n):
         else:
             # the window is n samples zero-padded to fftsize: the main lobe is fftsize/n bands wide
             assert abs(int(got[s]) - int(bands[s])) <= fftsize // n + 1, (s, got[s], bands[s])
-        if want_fn is not None:
-            # two float DFTs may order two bands differently only when those are equal to rounding
-            k = np.arange(1, nbands)[:, None] * np.arange(n)[None, :]
-            m = np.abs((w[None, :].astype(np.float64) * np.exp(-2j * np.pi * k / fftsize)).sum(1))
-            top = np.sort(m)[-2:]
-            if top[1] == 0 or (top[1] - top[0]) / top[1] > 1e-4:
-                assert got[s] == want_fn(rp.h, orc.fptr(w), n, 0.05), s
+        # two float DFTs may order two bands differently only when those are equal to rounding
+        k = np.arange(1, nbands)[:, None] * np.arange(n)[None, :]
+        m = np.abs((w[None, :].astype(np.float64) * np.exp(-2j * np.pi * k / fftsize)).sum(1))
+        top = np.sort(m)[-2:]
+        if top[1] == 0 or (top[1] - top[0]) / top[1] > 1e-4:
+            assert got[s] == rp.detect_carrier(w, n, 0.05), s
     # no offsets, threshold above everything
     none = mm.detect_carrier_batch(fftsize, d, n, 10.0)
     torch.cuda.synchronize()
@@ -672,7 +660,7 @@ def test_decode_batch_every_decoder(kind):
     assert total > 1000
     # independent of this repository's decoder source: the UNMODIFIED reference decoders (oracle/_ref/libfsk_ref.so,
     # src/databits_*.c, src/uic_codes.c) on the same records, for the decoders that keep no state between calls
-    if orc.have_ref() and kind in ("ascii8", "binary", "uic-ground", "uic-train"):
+    if kind in ("ascii8", "binary", "uic-ground", "uic-train"):
         for s in range(0, nstreams, 5):
             frames = []
             for r in rec[s, :nfr[s]]:

@@ -143,11 +143,10 @@ def test_binding_refuses_the_emulation_build():
     assert r.returncode != 0 and b"HOST-EMULATION" in r.stdout and b"refuses" in r.stdout
 
 
-def test_wav_locate_on_the_reference_transmitters_files(tmp_path):
+def test_wav_locate_on_the_reference_transmitters_files():
     """N2, the file side: the WAV images the reference's own transmitter writes (S16 by default,
     float32 with --float-samples) are located exactly; what is not mono PCM16/float32 is refused."""
     import struct
-    import subprocess
     import golden_util as gu
     g = gu.load("small-1200")
     a = gu.audio(refcases.BY_NAME["small-1200"], g)
@@ -168,10 +167,9 @@ def test_wav_locate_on_the_reference_transmitters_files(tmp_path):
     for bad in (b"", b"RIFFxxxxWAVX", wav(a, 48000, 1, 16, channels=2), wav(a, 48000, 1, 8), img[:30]):
         with pytest.raises(RuntimeError):
             mm.wav_locate(bad)
-    if orc.have_ref():                                         # a file written by the unmodified reference CLI
-        for extra, isfloat in (([], False), (["--float-samples"], True)):
-            path = str(tmp_path / "t.wav")
-            subprocess.run([orc.REF_CLI, "--tx", "--file", path, "1200"] + extra, input=b"wav header\n", check=True)
-            image = open(path, "rb").read()
-            off, n, rate, isf = mm.wav_locate(image)
-            assert rate == 48000 and isf == isfloat and off + n * (4 if isfloat else 2) == len(image)
+    # a file written by the unmodified reference CLI: its header as recorded, the samples' bytes zeroed
+    for extra, isfloat in (([], False), (["--float-samples"], True)):
+        head, size = orc.ref_cli_tx_image(["1200"] + extra, b"wav header\n")
+        image = head + bytes(size - len(head))
+        off, n, rate, isf = mm.wav_locate(image)
+        assert rate == 48000 and isf == isfloat and off + n * (4 if isfloat else 2) == len(image)

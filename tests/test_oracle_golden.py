@@ -43,7 +43,6 @@ def test_rx_restatement_matches_reference_calls(case):
         assert gu.close(ampl, cf[i, 2]), (i, ampl, cf[i, 2])
 
 
-@pytest.mark.ref
 @pytest.mark.parametrize("case", CASES, ids=IDS)
 def test_rx_restatement_decodes_and_reports_like_reference(case):
     g = gu.load(case["name"])

@@ -1,7 +1,7 @@
 """Pin the oracle's bit analyzer / frame search against (a) the raw FFT bins the
 unmodified reference computed on its own vectors (tests/golden, `bins`) and
 (b) oracle/_ref/libfsk_ref.so = the unmodified src/fsk.c compiled in place, on
-seeded noisy inputs.  CPU only."""
+seeded noisy inputs (its recorded answers where it is not built).  CPU only."""
 import numpy as np
 import pytest
 
@@ -82,7 +82,6 @@ def test_two_bin_dft_matches_reference_fft_bins(case):
     assert worst_noise < 2e-6, worst_noise
 
 
-@pytest.mark.ref
 @pytest.mark.parametrize("mode_name,kw", [("1200", {}), ("300", {}), ("rtty", dict(sample_rate=8000)),
                                           ("same", {}), ("12000", {}), ("rtty", {})])
 def test_find_frame_matches_compiled_reference_on_noisy_input(mode_name, kw):
